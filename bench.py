@@ -24,7 +24,13 @@ kernel (qb_comm.cu; consecutive steps are pipelined across GPUs), every rank end
 The default run (`--config all`) prints ONE JSON line: the C2 headline fields above plus `configs.{c3,c4,c5}` — the other
 BASELINE configs measured in the same process (each with value / e2e / roofline / parity / cpu_baseline): C3 10Mx768 SQ8 batch
 1024 on the int8 tensor cores, C4 one 6.25M-row PQ shard per GPU, C5 HNSW M=16 ef=128 with the traversal on the device.
-At N > 1 only the sharded configs (C2, C4) run.
+At N > 1 only the sharded configs (C2, C4) run.  --steps sets the number of timed steps of every config.
+
+`--dump-outputs DIR` writes, after the timed steps, the top-k lists each config's timed path returned in its last timed step:
+DIR/<config>_ids.npy (float64) and DIR/<config>_scores.npy (float32), [query, rank], -1 / NaN past a query's count.  Every
+input is generated from fixed seeds, so two builds run with the same arguments can be compared output for output.  C5 is
+left out: its graph comes from the multi-threaded builder, whose links depend on thread timing, so its lists vary from run
+to run.
 """
 from __future__ import annotations
 
@@ -66,7 +72,43 @@ def parse():
     ap.add_argument("--c5-rows", type=int, default=1_000_000, help="points of the HNSW index (BASELINE says 10M; the graph is built on the host cores inside the run)")
     ap.add_argument("--c5-queries", type=int, default=4096)
     ap.add_argument("--batch", type=int, default=1024, help="queries per batch (c3)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step of each config as DIR/<name>.npy")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
+
+
+# the top-k lists each config's timed path returned in its last timed step (--dump-outputs)
+OUTPUTS: dict[str, np.ndarray] = {}
+OUTPUTS_MAX_BYTES = 64 << 20
+
+
+def keep_lists(name: str, lists, top: int) -> None:
+    """Per-query ScoredPointOffset lists -> [query, rank] ids (float64: exact for any row id) and scores (float32)."""
+    ids = np.full((len(lists), top), -1.0, np.float64)
+    scores = np.full((len(lists), top), np.nan, np.float32)
+    for i, l in enumerate(lists):
+        ids[i, : l.size] = l["idx"]
+        scores[i, : l.size] = l["score"]
+    OUTPUTS[name + "_ids"], OUTPUTS[name + "_scores"] = ids, scores
+
+
+def device_lists(d_out, d_cnt):
+    """The lists a qb_*_search_batch_device call left in (d_out, d_cnt); the caller has synchronised the device."""
+    from qdrant_b200.scorer import SCORED_POINT_OFFSET
+
+    rec = d_out.cpu().numpy().view(SCORED_POINT_OFFSET)
+    cnt = d_cnt.cpu().numpy()
+    return [rec[i, : cnt[i]] for i in range(rec.shape[0])]
+
+
+def write_outputs(path: str) -> None:
+    total = sum(a.nbytes for a in OUTPUTS.values())
+    assert total <= OUTPUTS_MAX_BYTES, f"{total} bytes of outputs"
+    os.makedirs(path, exist_ok=True)
+    for name, a in OUTPUTS.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def ncu_traffic(name):
@@ -332,6 +374,7 @@ def main_ours(args):
     # sanity: the result of the last step must be a valid top-k
     last = searcher.results_host(1)[0]
     assert last.size == TOP and np.all(last["score"][:-1] >= last["score"][1:]), "invalid top-k from the timed region"
+    keep_lists("c2", [last], TOP)
 
     # ---- timed region 2: end to end through the public host API (H2D query, D2H results inside)
     for i in range(3):
@@ -474,7 +517,7 @@ def f32_batch_on(st, args, dev):
     torch.cuda.synchronize()
     st.search_stats(reset=True); st.profile_read(reset=True); st.profile(True)
     launches0 = int(lib().qb_kernel_launch_count())
-    K = 5
+    K = args.steps
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev0.record(stream)
     for _ in range(K):
@@ -485,10 +528,11 @@ def f32_batch_on(st, args, dev):
     launches = int(lib().qb_kernel_launch_count()) - launches0
     n_prof, prof_ms = st.profile_read(reset=True)
     st.profile(False)
+    keep_lists("f32_batch", device_lists(d_out, d_cnt), top)
     t0 = time.perf_counter()
-    for _ in range(3):
+    for _ in range(K):
         res = st.search_batch(queries, top)
-    e2e_ms = (time.perf_counter() - t0) * 1e3 / 3
+    e2e_ms = (time.perf_counter() - t0) * 1e3 / K
     searches, reruns = st.search_stats(reset=True)
     assert reruns == 0, f"f32 batch: {reruns} fallback reruns"
     qb.set_option("disable_mma", 1)
@@ -529,7 +573,6 @@ def main_c3(args):
     dev = torch.device("cuda", 0)
     torch.cuda.set_device(0)
     n, dim, nq, top = args.rows, args.dim, args.batch, TOP
-    args = argparse.Namespace(**dict(vars(args), steps=min(args.steps, 10)))   # a step is a 1024-query batch (~6 ms); 10 is plenty
     ad = dim + (16 - dim % 16) % 16
     chunk = 500_000
 
@@ -602,6 +645,7 @@ def main_c3(args):
     n_prof, prof_ms = st.profile_read(reset=True)
     st.profile(False)
     clk = clocks.stop()
+    keep_lists("c3", device_lists(d_out, d_cnt), top)
     for _ in range(2):
         st.search_batch(queries, top)
     t0 = time.perf_counter()
@@ -693,7 +737,6 @@ def main_c4(args):
     from qdrant_b200.sharded import ShardedSegmentSearcher
 
     world, rank, local_rank, dev = dist_ctx()
-    args = argparse.Namespace(**dict(vars(args), steps=min(args.steps, 5)))   # a step is a 256-query batch over the shard
     total_rows, dim, chunk, nq, top = 50_000_000, 1536, 16, 256, TOP
     if args.rows != N_ROWS:
         total_rows = args.rows
@@ -740,6 +783,7 @@ def main_c4(args):
     n_prof, prof_ms = st.profile_read(reset=True)
     st.profile(False)
     clk = clocks.stop() if rank == 0 else None
+    keep_lists("c4", searcher.results_host(nq), top)
     for _ in range(2):
         searcher.search(queries)
     barrier()
@@ -868,7 +912,7 @@ def main_c5(args):
     def step_device():
         check(lib().qb_hnsw_search_batch_device(hg._h, vp(d_q.data_ptr()), nq, top, ef, entry, entry_level, vp(d_out.data_ptr()), vp(d_cnt.data_ptr())))
 
-    W, K = 3, max(3, min(args.steps, 10))
+    W, K = 3, args.steps
     for _ in range(W):
         step_device()
     torch.cuda.synchronize()
@@ -965,6 +1009,8 @@ def main_all(args):
         if extras:
             line["configs"] = extras
         print(json.dumps(line))
+    if rank == 0 and args.dump_outputs:
+        write_outputs(args.dump_outputs)
     sys.stdout.flush()
     if world > 1:
         dist.barrier()

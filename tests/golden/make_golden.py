@@ -11,6 +11,11 @@ Contents
     e2e_*                                            a 256 x 768 SQ8 cosine segment, 3 f32 queries, and the scores
                                                      postprocess_score(impl_score_dot_avx(query code, row code)) of every (query, row)
     bq_*                                             one-bit rows, scalar-8/4-bit and binary queries, impl_xor_popcnt_* outputs
+
+and tests/golden/ref_kernels_kat.npz: the same kernels' results on the seeded inputs the tests regenerate themselves
+    sq8_{dot_avx,l1_avx,dot_sse}[c]     impl_score_* on case c of tests.test_oracle_kat.sq8_kat_codes()
+    bq_xor_{s8,s4,bin}[c, row]          impl_xor_popcnt_{scalar8_avx,scalar4_avx,sse}_uint128 on tests.test_oracle_kat.bq_kat_vectors()
+    sq8_e2e_scores[query, row]          postprocess_score(impl_score_dot_avx) on test_gpu_quant.test_sq8_matches_reference_c_kernel's segment
 """
 import ctypes as C
 import os
@@ -84,5 +89,46 @@ def main():
     print(path, os.path.getsize(path), "bytes")
 
 
+def ref_kernels_kat():
+    from oracle import oracle as o
+    from qdrant_b200 import scorer as qb
+    from tests.test_gpu_quant import gen
+    from tests.test_oracle_kat import REF_KAT, bq_kat_vectors, sq8_kat_codes
+
+    R = o.ref()
+    assert R is not None, "oracle/_ref/libsimd_utils.so is needed to generate the golden vectors"
+    u8p = C.POINTER(C.c_uint8)
+    out = {"sq8_" + name: [] for name in ("dot_avx", "l1_avx", "dot_sse")}
+    for dim, q, v in sq8_kat_codes():
+        for name in ("dot_avx", "l1_avx", "dot_sse"):
+            out["sq8_" + name].append(getattr(R, "impl_score_" + name)(q.ctypes.data_as(u8p), v.ctypes.data_as(u8p), dim))
+    out = {k: np.array(x, np.float32) for k, x in out.items()}
+
+    xor = {"s8": [], "s4": [], "bin": []}
+    for dim, data, q in bq_kat_vectors():
+        for tag, qenc, fn in (("s8", o.BQQ_SCALAR8, R.impl_xor_popcnt_scalar8_avx_uint128), ("s4", o.BQQ_SCALAR4, R.impl_xor_popcnt_scalar4_avx_uint128),
+                              ("bin", o.BQQ_SAME, R.impl_xor_popcnt_sse_uint128)):
+            bq = o.BQ.encode(data, o.BQ_ONE, qenc, o.QD_DOT, False)
+            qe = bq.encode_query(q)
+            words = bq.rows.shape[1] // 16
+            xor[tag].append([fn(qe.ctypes.data_as(u8p), np.ascontiguousarray(bq.rows[i]).ctypes.data_as(u8p), words) for i in range(data.shape[0])])
+    out.update({"bq_xor_" + tag: np.array(x, np.uint32) for tag, x in xor.items()})
+
+    base, queries = gen(o, qb, qb.Distance.Cosine, 256, 768)
+    sq = o.SQ8.encode(base, o.QD_DOT, False)
+    scores = np.zeros((queries.shape[0], 256), np.float32)
+    for qi, q in enumerate(queries):
+        code, off = sq.encode_query(o.preprocess_f32(o.COSINE, q))
+        for i in range(256):
+            row = np.ascontiguousarray(sq.rows[i])
+            raw = np.float32(R.impl_score_dot_avx(code.ctypes.data_as(u8p), row[4:].ctypes.data_as(u8p), 768))
+            voff = row[:4].view(np.float32)[0]
+            scores[qi, i] = np.float32(np.float32(np.float32(sq.meta.multiplier) * raw) + off) + voff   # encoded_vectors_u8.rs:101-103
+    out["sq8_e2e_scores"] = scores
+    np.savez_compressed(REF_KAT, **out)
+    print(REF_KAT, os.path.getsize(REF_KAT), "bytes")
+
+
 if __name__ == "__main__":
     main()
+    ref_kernels_kat()

@@ -62,26 +62,20 @@ def test_sq8_scores_bit_exact(qb, oracle, dist, n, dim):
 
 
 def test_sq8_matches_reference_c_kernel(qb, oracle):
-    """End-to-end against the reference's OWN impl_score_dot_avx (oracle/_ref) + postprocess_score."""
-    import ctypes as C
+    """End-to-end against the reference's OWN impl_score_dot_avx + postprocess_score: its scores of these queries and rows,
+    multiplier * raw + query offset + row offset, are stored in tests/golden/ref_kernels_kat.npz."""
+    from tests.test_oracle_kat import REF_KAT
 
-    R = oracle.ref()
-    if R is None:
-        pytest.skip("oracle/_ref/libsimd_utils.so not available")
+    want = np.load(REF_KAT)["sq8_e2e_scores"]
     d = qb.Distance.Cosine
     base, queries = gen(oracle, qb, d, 256, 768)
     sq = oracle.SQ8.encode(base, oracle.QD_DOT, False)
     st = qb.ScalarQuantizedVectors(sq.rows, 768, sq.meta.alpha, sq.meta.offset, sq.meta.multiplier, d)
-    u8p = C.POINTER(C.c_uint8)
-    for q in queries:
-        code, off = sq.encode_query(oracle.preprocess_f32(oracle.COSINE, q))
+    assert want.shape == (queries.shape[0], 256)
+    for qi, q in enumerate(queries):
         got = st.raw_scorer(q).score_points(np.arange(256, dtype=np.uint32))
         for i in range(256):
-            row = np.ascontiguousarray(sq.rows[i])
-            raw = np.float32(R.impl_score_dot_avx(code.ctypes.data_as(u8p), row[4:].ctypes.data_as(u8p), 768))
-            voff = row[:4].view(np.float32)[0]
-            want = np.float32(np.float32(np.float32(sq.meta.multiplier) * raw) + off) + voff
-            assert got[i] == want
+            assert got[i] == want[qi, i], (qi, i)
     st.close()
 
 

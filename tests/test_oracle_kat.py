@@ -5,12 +5,15 @@ Each case re-types the fixed vectors of a reference unit test and asserts what t
   f32 : lib/segment/src/spaces/simple_avx.rs:218-256, simple_sse.rs:206-..., simple.rs:248-277
   u8  : lib/segment/src/spaces/metric_uint/avx2/{dot.rs:77-106,cosine.rs:112-170,euclid.rs,manhattan.rs}
   topk: lib/segment/src/spaces/tools.rs:64-75
-  SQ8/BQ inner loops: the reference's C kernels compiled verbatim (oracle/_ref/libsimd_utils.so)
+  SQ8/BQ inner loops: the reference's C kernels compiled verbatim (oracle/_ref/libsimd_utils.so); their results on the
+        seeded inputs below are stored in tests/golden/ref_kernels_kat.npz (tests/golden/make_golden.py)
 """
 import ctypes as C
+import os
 
 import numpy as np
-import pytest
+
+REF_KAT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_kernels_kat.npz")
 
 
 def f32_kat():
@@ -117,13 +120,8 @@ def test_topk_matches_sort(oracle):
     np.testing.assert_array_equal(res["idx"], order.astype(np.uint32))
 
 
-def test_sq8_inner_loops_match_reference_c(oracle):
-    """oracle restatement == the reference's own avx2.c / sse.c compiled verbatim, on random + extreme codes."""
-    R = oracle.ref()
-    if R is None:
-        pytest.skip("oracle/_ref/libsimd_utils.so not built (no /root/reference and no prebuilt)")
-    L = oracle.lib()
-    u8p = C.POINTER(C.c_uint8)
+def sq8_kat_codes():
+    """(dim, query code, row code): random and extreme 7-bit codes, seeded."""
     rng = np.random.default_rng(42)
     for dim in (16, 32, 48, 64, 80, 768, 784, 1536, 4096):
         for trial in range(20):
@@ -133,44 +131,54 @@ def test_sq8_inner_loops_match_reference_c(oracle):
                 q[:] = 127; v[:] = 127
             if trial == 1:
                 q[:] = 0
-            qp, vp = q.ctypes.data_as(u8p), v.ctypes.data_as(u8p)
-            assert L.qo_sq8_dot_avx(qp, vp, dim) == R.impl_score_dot_avx(qp, vp, dim)
-            assert L.qo_sq8_l1_avx(qp, vp, dim) == R.impl_score_l1_avx(qp, vp, dim)
-            # the SSE tier is the same integers for dims whose sums stay < 2^24 (exactness window)
-            if dim <= 1040:
-                assert R.impl_score_dot_sse(qp, vp, dim) == R.impl_score_dot_avx(qp, vp, dim)
-                assert R.impl_score_dot_avx(qp, vp, dim) == np.float32(int(np.dot(q.astype(np.int64), v.astype(np.int64))))
+            yield dim, q, v
 
 
-def test_bq_popcount_matches_reference_c(oracle):
-    R = oracle.ref()
-    if R is None:
-        pytest.skip("oracle/_ref/libsimd_utils.so not built")
+def bq_kat_vectors():
+    """(dim, 4 stored f32 vectors, f32 query), seeded."""
     rng = np.random.default_rng(9)
-    u8p = C.POINTER(C.c_uint8)
     for dim in (1, 127, 128, 129, 768, 1000, 1536):
         data = rng.standard_normal((4, dim)).astype(np.float32)
         q = rng.standard_normal(dim).astype(np.float32)
-        for qenc, bits, fn in ((oracle.BQQ_SCALAR8, 8, R.impl_xor_popcnt_scalar8_avx_uint128),
-                               (oracle.BQQ_SCALAR4, 4, R.impl_xor_popcnt_scalar4_avx_uint128)):
+        yield dim, data, q
+
+
+def test_sq8_inner_loops_match_reference_c(oracle):
+    """oracle restatement == the reference's own avx2.c / sse.c compiled verbatim, on random + extreme codes."""
+    R = np.load(REF_KAT)
+    L = oracle.lib()
+    u8p = C.POINTER(C.c_uint8)
+    for c, (dim, q, v) in enumerate(sq8_kat_codes()):
+        qp, vp = q.ctypes.data_as(u8p), v.ctypes.data_as(u8p)
+        assert L.qo_sq8_dot_avx(qp, vp, dim) == R["sq8_dot_avx"][c], (c, dim)
+        assert L.qo_sq8_l1_avx(qp, vp, dim) == R["sq8_l1_avx"][c], (c, dim)
+        # the SSE tier is the same integers for dims whose sums stay < 2^24 (exactness window)
+        if dim <= 1040:
+            assert R["sq8_dot_sse"][c] == R["sq8_dot_avx"][c]
+            assert R["sq8_dot_avx"][c] == np.float32(int(np.dot(q.astype(np.int64), v.astype(np.int64)))), (c, dim)
+    assert R["sq8_dot_avx"].size == c + 1
+
+
+def test_bq_popcount_matches_reference_c(oracle):
+    R = np.load(REF_KAT)
+    for c, (dim, data, q) in enumerate(bq_kat_vectors()):
+        for qenc, bits, tag in ((oracle.BQQ_SCALAR8, 8, "s8"), (oracle.BQQ_SCALAR4, 4, "s4")):
             bq = oracle.BQ.encode(data, oracle.BQ_ONE, qenc, oracle.QD_DOT, False)
             qe = bq.encode_query(q)
-            words = bq.rows.shape[1] // 16
             for i in range(data.shape[0]):
-                row = np.ascontiguousarray(bq.rows[i])
-                x = fn(qe.ctypes.data_as(u8p), row.ctypes.data_as(u8p), words)
+                x = int(R["bq_xor_" + tag][c, i])      # impl_xor_popcnt_scalar{8,4}_avx_uint128(query, row i)
                 xf = np.float32(x) / np.float32((1 << bits) - 1)
                 zeros = np.float32(dim) - xf
                 assert bq.score(qe, i) == zeros - xf
         bq = oracle.BQ.encode(data, oracle.BQ_ONE, oracle.BQQ_SAME, oracle.QD_DOT, False)
         qe = bq.encode_query(q)
         for i in range(data.shape[0]):
-            row = np.ascontiguousarray(bq.rows[i])
-            x = R.impl_xor_popcnt_sse_uint128(qe.ctypes.data_as(u8p), row.ctypes.data_as(u8p), bq.rows.shape[1] // 16)
+            x = int(R["bq_xor_bin"][c, i])              # impl_xor_popcnt_sse_uint128(query, row i)
             assert bq.score(qe, i) == np.float32(dim - x) - np.float32(x)
             bits_q = (q > 0)
             bits_v = (data[i] > 0)
             assert x == int(np.sum(bits_q != bits_v))
+    assert R["bq_xor_bin"].shape[0] == c + 1
 
 
 def test_f16_avx_vs_scalar_tolerance(oracle):
